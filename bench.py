@@ -2,6 +2,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA engine)
     python bench.py --impl reference --gpus N --steps K ...  # CPU arm (oracle port, host cores)
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's outputs as DIR/*.npy
 
 A "step" is one pass of the hot path over one batch of synthetic input:
 ``flow(c).log_prob(x)`` + the fixed-order sum of the log-densities (the per-device term of
@@ -486,8 +487,7 @@ def run_ours(args) -> None:
 
     def step(i: int):
         d = flow(cs[i % NBUF])
-        lp, _ = d.log_prob_and_sum(xs[i % NBUF], sum_out=ring.slot(B))
-        return lp
+        return d.log_prob_and_sum(xs[i % NBUF], sum_out=ring.slot(B))
 
     with torch.no_grad():
         # ---- parity of the bench workload against the oracle (small slice, outside timing)
@@ -518,10 +518,12 @@ def run_ours(args) -> None:
             torch.cuda.synchronize()
             e0.record()
             for i in range(args.steps):
-                step(i)
+                lp, lp_sum = step(i)
             nll_means = ring.means()  # waits for the outstanding mean-NLL collectives: inside the timed region
             e1.record()
             torch.cuda.synchronize()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"log_prob": lp, "log_prob_sum": lp_sum, "mean_nll": nll_means[-1:]})
         if world > 1:
             dist.barrier()
         elapsed_ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
@@ -616,6 +618,23 @@ def run_ours(args) -> None:
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_ROWS = 15 << 20  # 60 MiB of float32 log-densities: a dump stays under 64 MB
+
+
+def dump_outputs(out_dir: str, outputs: dict) -> None:
+    """Writes what the last timed step returned (rank 0) as out_dir/<name>.npy, in the dtype it was
+    computed in (float32 / float64), so that two builds can be compared output for output on the same
+    seeded inputs.  Of a batch over DUMP_ROWS rows, a fixed, seeded sample of DUMP_ROWS rows is kept
+    (the same rows in every run with the same --batch)."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, t in outputs.items():
+        a = t.detach().cpu().numpy()
+        if a.shape[0] > DUMP_ROWS:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], DUMP_ROWS, replace=False))]
+        np.save(out / f"{name}.npy", a)
 
 
 def time_training_step(flow, x, c, rows: int, iters: int) -> dict:
@@ -772,7 +791,12 @@ def main() -> None:
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-training-step", action="store_true", help="skip the forward+backward timing (extra object)")
     ap.add_argument("--no-configs", action="store_true", help="skip the cfg3 / cfg4 / cfg5 entries of the line")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the engine arm; the reference arm keeps none")
     if args.impl == "reference":
         run_reference(args)
     else:

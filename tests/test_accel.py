@@ -1,67 +1,32 @@
 """`zuko_b200.accelerate(flow)` — the drop-in seam of SURVEY §8(b): an engine-backed
 LazyDistribution that shares the parameters / buffers of an existing flow.
 
-CPU part: structure, sharing and error behaviour, against flows built by the *unmodified
-reference* when it is importable in this container (it is not on the GPU box) and against the
-engine's own modules otherwise.  GPU part: the accelerated flow reproduces the golden
+CPU part: structure, sharing and error behaviour, against flows built by the constructors of the
+*unmodified reference* (rebuilt from their recorded module trees, tests/golden/make_golden_accel.py)
+and against the engine's own modules.  GPU part: the accelerated flow reproduces the golden
 log-densities and follows in-place updates of the source flow.
 """
 
 from __future__ import annotations
 
-import os
-import sys
-from functools import partial
-
+import numpy as np
 import pytest
 import torch
 
 import zuko_b200
 from zuko_b200.accel import _convert, _share
 
-from cases import SMALL_CASES, assert_log_prob_parity, build_flow, load
+from cases import GOLDEN, SMALL_CASES, assert_log_prob_parity, build_flow, load
+from module_tree import rebuild
 
-REFERENCE = "/root/reference"
-
-
-def _reference():
-    if not os.path.isdir(os.path.join(REFERENCE, "zuko")):
-        pytest.skip("reference sources are not present on this machine")
-    sys.dont_write_bytecode = True
-    if REFERENCE not in sys.path:
-        sys.path.append(REFERENCE)
-    import zuko
-
-    return zuko
+REJECTED = ("maf_prelu", "naf", "gf", "maf_float64")  # options the engine does not implement
 
 
-def _reference_flows(zuko):
-    torch.manual_seed(0)
-    F, T, D = zuko.flows, zuko.transforms, zuko.distributions
-    base = lambda n: F.UnconditionalDistribution(D.DiagNormal, torch.zeros(n), torch.ones(n), buffer=True)  # noqa: E731
-    adjacency = torch.tensor([[1, 0, 0], [1, 1, 0], [0, 1, 1]], dtype=bool)
-    return {
-        "nsf": F.NSF(5, 3, transforms=2, bins=4, hidden_features=[32, 32]),
-        "maf": F.MAF(4, 0, transforms=2, hidden_features=[16]),
-        "maf_randperm": F.MAF(6, 2, transforms=3, randperm=True),
-        "nice": F.NICE(5, 2, transforms=3),
-        "nsf_passes2": F.NSF(6, 0, transforms=2, passes=2),
-        "nsf_single_feature": F.NSF(1, 2, transforms=2),
-        "ncsf": F.NCSF(3, 2, transforms=2, bins=4, hidden_features=[16]),
-        "maf_elu": F.MAF(4, 2, transforms=2, hidden_features=[32, 32], activation=torch.nn.ELU),
-        "nsf_residual": F.NSF(4, 2, transforms=2, hidden_features=[16, 32, 32], residual=True),
-        "adjacency": F.Flow([F.MaskedAutoregressiveTransform(3, 1, adjacency=adjacency)], base(3)),
-        "composed": F.Flow(
-            [
-                F.UnconditionalTransform(T.SoftclipTransform, bound=6.0),
-                F.MaskedAutoregressiveTransform(4, 2, univariate=partial(T.MonotonicRQSTransform, slope=1e-2), shapes=[(8,), (8,), (7,)]),
-                F.UnconditionalTransform(T.PermutationTransform, torch.randperm(4), buffer=True),
-                F.UnconditionalTransform(T.RotationTransform, torch.randn(4, 4)),
-                F.GeneralCouplingTransform(4, 2).inv,
-            ],
-            base(4),
-        ),
-    }  # fmt: skip
+def _reference_flows():
+    """Fresh copies of the reference-built flows: the reference's class names, constructor attributes,
+    masks, orders and state-dict layout (tests/module_tree.py)."""
+    with np.load(GOLDEN / "accel_reference_flows.npz") as payload:
+        return rebuild(payload)
 
 
 def _assert_shared(acc, src):
@@ -76,8 +41,9 @@ def _assert_shared(acc, src):
 
 
 def test_accelerate_reference_flows_share_tensors():
-    zuko = _reference()
-    for name, src in _reference_flows(zuko).items():
+    for name, src in _reference_flows().items():
+        if name in REJECTED:
+            continue
         acc = zuko_b200.accelerate(src)
         assert isinstance(acc, zuko_b200.lazy.LazyDistribution), name
         _assert_shared(acc, src)
@@ -87,21 +53,19 @@ def test_accelerate_reference_flows_share_tensors():
 
 
 def test_accelerate_keeps_reference_built_masks_and_orders():
-    zuko = _reference()
-    src = _reference_flows(zuko)["maf_randperm"]
+    src = _reference_flows()["maf_randperm"]
     acc = zuko_b200.accelerate(src)
     for ts, ta in zip(src.transform.transforms, acc.transform.transforms, strict=True):
         assert ta.passes == ts.passes and torch.equal(ta.order, ts.order)
         for ms, ma in zip(ts.hyper, ta.hyper, strict=True):
             if hasattr(ms, "mask"):
                 assert ma.mask is ms.mask
-    adj = zuko_b200.accelerate(_reference_flows(zuko)["adjacency"])
+    adj = zuko_b200.accelerate(_reference_flows()["adjacency"])
     assert adj.transform.transforms[0].order is None and adj.transform.transforms[0].passes == 3
 
 
 def test_accelerate_sees_updates_of_the_source():
-    zuko = _reference()
-    src = _reference_flows(zuko)["nsf"]
+    src = _reference_flows()["nsf"]
     acc = zuko_b200.accelerate(src)
     layer = acc.transform.transforms[0]
     sig0 = layer._layer_signature()
@@ -119,13 +83,12 @@ def test_accelerate_sees_updates_of_the_source():
 
 
 def test_accelerate_rejects_what_the_engine_does_not_implement():
-    zuko = _reference()
-    F = zuko.flows
-    for bad in (F.MAF(3, 0, activation=torch.nn.PReLU), F.NAF(3, 0), F.GF(3, 0)):
+    flows = _reference_flows()
+    for bad in ("maf_prelu", "naf", "gf"):
         with pytest.raises(NotImplementedError, match="accelerate"):
-            zuko_b200.accelerate(bad)
+            zuko_b200.accelerate(flows[bad])
     with pytest.raises(TypeError, match="float32"):
-        zuko_b200.accelerate(F.MAF(3, 0).double())
+        zuko_b200.accelerate(flows["maf_float64"])
     with pytest.raises(TypeError, match="lazy Flow"):
         zuko_b200.accelerate(torch.nn.Linear(2, 2))
 

@@ -7,6 +7,8 @@ import subprocess
 import sys
 from pathlib import Path
 
+import pytest
+
 ROOT = Path(__file__).resolve().parent.parent
 
 
@@ -32,8 +34,6 @@ def test_engine_arm_refuses_without_cuda():
     import torch
 
     if torch.cuda.is_available():
-        import pytest
-
         pytest.skip("this check is for the CPU-only build container")
     r = _run("--steps", "1")
     assert r.returncode != 0 and "no CUDA device" in (r.stderr + r.stdout)
@@ -63,3 +63,57 @@ def test_tensor_roofline_denominator_follows_the_clock():
     peak, kind = bench.tensor_peak(peaks, {"sm_mhz": 1680.0, "sm_max_mhz": 1965.0, "reasons": ["sw_power_cap"]})
     assert abs(peak - 1640.0 * 1680.0 / 1965.0) < 1e-9 and "1680" in kind and "burst" in kind
     assert bench.tensor_peak(peaks, {}) == (1640.0, "burst")  # no NVML: nothing to scale by
+
+
+def test_dump_outputs_keeps_dtypes_and_a_fixed_sample(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+
+    sys.path.insert(0, str(ROOT))
+    import bench
+
+    monkeypatch.setattr(bench, "DUMP_ROWS", 8)
+    outputs = {"log_prob": torch.arange(20, dtype=torch.float32), "log_prob_sum": torch.tensor([190.0], dtype=torch.float64)}
+    bench.dump_outputs(str(tmp_path / "a"), outputs)
+    bench.dump_outputs(str(tmp_path / "b"), outputs)
+    lp, total = np.load(tmp_path / "a" / "log_prob.npy"), np.load(tmp_path / "a" / "log_prob_sum.npy")
+    assert lp.dtype == np.float32 and lp.shape == (8,) and np.all(np.diff(lp) > 0) and set(lp) <= set(range(20))
+    assert total.dtype == np.float64 and total.tolist() == [190.0]
+    assert np.array_equal(lp, np.load(tmp_path / "b" / "log_prob.npy"))
+
+
+def test_bench_rejects_bad_arguments():
+    assert "--steps" in _run("--steps", "0").stderr
+    assert "--dump-outputs" in _run("--impl", "reference", "--dump-outputs", "x").stderr
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_timed_step(device, tmp_path):
+    """The dumped log-densities are those of the seeded input buffer the last timed step used (the fp64
+    oracle on the same rows), and two runs dump identical outputs."""
+    import numpy as np
+    import torch
+
+    sys.path.insert(0, str(ROOT))
+    import bench
+    from oracle import oracle
+
+    B, steps = 4096, 3
+    for run in ("a", "b"):
+        r = _run("--batch", str(B), "--steps", str(steps), "--warmup", "1", "--no-configs", "--no-training-step",
+                 "--no-cpu-baseline", "--dump-outputs", str(tmp_path / run))  # fmt: skip
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout.splitlines()[-1])["steps"] == steps
+    lp = np.load(tmp_path / "a" / "log_prob.npy")
+    assert lp.dtype == np.float32 and lp.shape == (B,)
+    g = torch.Generator().manual_seed(1234)
+    xs = [torch.randn(B, bench.D, generator=g) for _ in range(4)]  # bench.run_ours: x buffers, then c buffers
+    cs = [torch.randn(B, bench.C, generator=g) for _ in range(4)]
+    x, c = xs[(steps - 1) % 4], cs[(steps - 1) % 4]
+    ref = oracle.flowspec_from_module(bench.build_model()).log_prob(x.numpy(), c.numpy())
+    assert np.max(np.abs(lp - ref) / np.maximum(np.abs(ref), 1.0)) < 1e-5
+    total = np.load(tmp_path / "a" / "log_prob_sum.npy")
+    assert total.dtype == np.float64 and abs(total[0] - lp.astype(np.float64).sum()) < 1e-6 * np.abs(lp).sum()
+    assert np.array_equal(lp, np.load(tmp_path / "b" / "log_prob.npy"))
+    assert np.array_equal(total, np.load(tmp_path / "b" / "log_prob_sum.npy"))
+    assert np.load(tmp_path / "a" / "mean_nll.npy").tolist() == [-total[0] / B]
