@@ -61,18 +61,18 @@ void zk_debug_timeline(long long* device_buffer) { zk::g_timeline = device_buffe
 int zk_debug_wide_schedule(int n_linear, const int* dims, const uint8_t* const* masks_host, int univariate, int bins,
                            int features, int context, uint32_t* out_items, int max_items, uint32_t* out_rd_mask,
                            int* out_perm) {
-    return zk::wide_schedule_host(n_linear, dims, masks_host, univariate, bins, features, context, out_items, max_items,
+    return zk::pair_schedule_host(1, n_linear, dims, masks_host, univariate, bins, features, context, out_items, max_items,
                                   out_rd_mask, out_perm);
 }
 int zk_debug_dual_schedule(int n_linear, const int* dims, const uint8_t* const* masks_host, int univariate, int bins,
                            int features, int context, uint32_t* out_items, int max_items, uint32_t* out_rd_mask,
                            int* out_perm) {
-    return zk::dual_schedule_host(n_linear, dims, masks_host, univariate, bins, features, context, out_items, max_items,
+    return zk::pair_schedule_host(2, n_linear, dims, masks_host, univariate, bins, features, context, out_items, max_items,
                                   out_rd_mask, out_perm);
 }
 int zk_debug_watchdog_read(uint32_t* out, int n_words) {
     if (!zk::g_watch_host || !out || n_words <= 0) return 0;
-    const int n = n_words < 1024 ? n_words : 1024;
+    const int n = n_words < zk::W_WATCH_WORDS ? n_words : zk::W_WATCH_WORDS;
     for (int i = 0; i < n; ++i) out[i] = ((volatile uint32_t*)zk::g_watch_host)[i];
     return n;
 }
@@ -464,8 +464,14 @@ int zk_layer_fused_info(const zk_layer* l, double* out) {
     if (!pk || l->circ || !fused_layer_supported(m, l->uni, l->K, l->D, l->C)) return 0;
     const int kind = fused_layer_kind(m, l->uni, l->K, l->D, l->C);
     out[0] = kind;
-    out[1] = kind == 3 ? pk->dual.n_items : (kind == 2 ? pk->wide.n_items : pk->fused.n_items);
-    out[2] = kind == 3 ? pk->dual.issued_macs_per_row : (kind == 2 ? pk->wide.issued_macs_per_row : pk->fused.issued_macs_per_row);
+    if (kind == 1) {
+        out[1] = pk->fused.n_items;
+        out[2] = pk->fused.issued_macs_per_row;
+    } else {
+        const WidePack& wp = (kind == 3) ? pk->dual : pk->wide;
+        out[1] = wp.n_items;
+        out[2] = wp.issued_macs_per_row;
+    }
     return kind;
 }
 

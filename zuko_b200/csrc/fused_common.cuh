@@ -1,6 +1,6 @@
-// zuko_b200 — device helpers shared by the two fully fused layer kernels
-// (fused_layer.cu: hidden width <= 256, one CTA per tile; fused_wide.cu: hidden width <= 512,
-// CTA pairs on cta_group::2 MMAs) and the host-side preparation they have in common.
+// zuko_b200 — device helpers shared by the fully fused layer kernels
+// (fused_layer.cu: hidden width <= 256, one CTA per tile; fused_wide.cu / fused_dual.cu: CTA pairs on
+// cta_group::2 MMAs) and the host-side preparation they have in common (fused_layer.cu, fused_plan.cu).
 #pragma once
 
 #include <type_traits>
@@ -79,5 +79,20 @@ struct FusedHostPrep {
 void fused_degree_perm(const int* dims, int L, const std::vector<std::vector<uint8_t>>& Mk,
                        std::vector<std::vector<int>>& perm);
 zk_status fused_host_prepare(zk_mlp* m, const uint8_t* const* mask_dev, FusedPack& f, FusedHostPrep& hp);
+
+// Which (chunk, K block) tiles of the degree-permuted masked matrices hold a non-zero weight.  Hidden
+// layers are cut into chunks of `cw` rows (64 or 128), the output layer into ceil(D / DPC) chunks of
+// DPC dims (DPC * P rows).
+struct FusedTileMap {
+    std::vector<std::vector<uint32_t>> kbmask;  // [layer][chunk]: bit kb = K block kb is read (at least bit 0)
+    std::vector<std::vector<int>> kmax;         // [layer][chunk * 8 + kb]: last column of the block any row of the chunk reads
+};
+FusedTileMap fused_tile_map(const int* dims, int L, const std::vector<std::vector<uint8_t>>& Mk,
+                            const std::vector<std::vector<int>>& perm, int cw, int univariate, int bins, int D);
+// Builds the pack `wp` of a pair kernel with S sub-tiles per CTA (pk->wide: S = 1, pk->dual: S = 2):
+// tensor maps, issue schedule and its bookkeeping.  wp.ready stays false when the dry run rejects the
+// schedule.  The shape is the caller's to check.
+zk_status fused_pair_prepare(zk_mlp* m, const uint8_t* const* mask_dev, int univariate, int bins, int D, int C,
+                             WidePack& wp, int S);
 
 }  // namespace zk

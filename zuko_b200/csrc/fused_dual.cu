@@ -24,10 +24,7 @@
 // Warp roles as in fused_wide.cu: warp 0 W producer (both CTAs), warp 1 MMA issuer and warp 2 scout
 // (leader CTA), warps 4-19 epilogue.
 
-#include <string.h>
-
 #include <algorithm>
-#include <atomic>
 
 #include "activations.cuh"
 #include "fused_common.cuh"
@@ -54,12 +51,8 @@ constexpr uint32_t D_AUX_BYTES = D_BAR_SLOTS * 8 + 2 * 2 * DM * 4; // + ladj par
 constexpr uint32_t D_SMEM_MAX = 232448;
 constexpr uint32_t TMD_D = 256;                                    // first accumulator column
 
-// schedule entry (uint2): x = flags, y = first weight row of the chunk
-//   x [1:0] K block | [2] sub-tile | [3] first K block of its chunk | [4] last K block of its chunk |
-//     [5] first read of this sub-tile's A block in this layer (wait a_ready) | [6] last read (commit a_free) |
-//     [7] output layer | [15:8] a_ready phases (index = 4 sub-tile + kb) consumed without reading |
-//     [18:16] layer | [21:20] trailing 16-column MMA steps that are all-zero for this chunk (not issued)
-constexpr uint32_t DS_FIRST = 8u, DS_LAST = 16u, DS_AWAIT = 32u, DS_AFREE = 64u, DS_OUT = 128u;
+// schedule entries: pair_common.cuh (S = 2: bits [1:0] are the K block, bit 2 the sub-tile)
+constexpr uint32_t DS_FIRST = WS_FIRST, DS_LAST = WS_LAST, DS_AWAIT = WS_AWAIT, DS_AFREE = WS_AFREE, DS_OUT = WS_OUT;
 
 struct DualParams {
     CUtensorMap mapW[ZK_FUSED_MAX_LINEAR];
@@ -572,341 +565,29 @@ zk_status launch_dual_t(const DualParams& p, bool fast, int grid, size_t smem, c
     return go(fused_dual_kernel<UNI, KT, false, false, false>);
 }
 
-struct DualShape {
-    int L, nch, KB0, KBH, n_last;
-};
-
-// Replays the kernel's barrier protocol on the schedule of one pair tile (three tiles back to back;
-// MMA completions immediate): MMA side, epilogue group 0, epilogue group 1.  Rejects schedules that
-// deadlock or let an mbarrier run two phases ahead of its waiter.
-bool dual_dry_run(const std::vector<uint2>& items, const uint32_t* rd_mask, const DualShape& sh, int policy) {
-    const int n = (int)items.size();
-    const int TILES = 3;
-    int d_full[2] = {0, 0}, d_empty[2] = {0, 0}, a_ready[8] = {0}, a_free[8] = {0};
-    int d_full_seen[2] = {0, 0}, d_empty_seen[2] = {0, 0}, a_ready_seen[8] = {0}, a_free_seen[8] = {0};
-    bool ok = true;
-    auto complete = [&](int* done, const int* seen, int idx) {
-        if (done[idx] != seen[idx]) ok = false;
-        done[idx]++;
-    };
-    int mi = 0;
-    int cnt[2] = {0, 0};
-    auto mma_step = [&]() -> bool {
-        if (mi >= TILES * n) return false;
-        const uint32_t it = items[mi % n].x;
-        const int u = (int)((it >> 2) & 1u);
-        if ((it & DS_FIRST) && d_empty[u] < cnt[u]) return false;
-        for (int k2 = 0; k2 < 8; ++k2)
-            if (((it >> (8 + k2)) & 1u) && a_ready[k2] <= a_ready_seen[k2]) return false;
-        const int kb8 = 4 * u + (int)(it & 3u);
-        if ((it & DS_AWAIT) && a_ready[kb8] <= a_ready_seen[kb8]) return false;
-        if (it & DS_FIRST) { d_empty_seen[u] = cnt[u]; ++cnt[u]; }
-        for (int k2 = 0; k2 < 8; ++k2)
-            if ((it >> (8 + k2)) & 1u) a_ready_seen[k2]++;
-        if (it & DS_AWAIT) a_ready_seen[kb8]++;
-        if (it & DS_AFREE) complete(a_free, a_free_seen, kb8);
-        if (it & DS_LAST) complete(d_full, d_full_seen, u);
-        ++mi;
-        return true;
-    };
-    struct Step { int kind, a; };  // 0 stage, 1 wait d_full(k-th chunk), 2 drain, 3 wait a_free(kb), 4 write(ch)
-    std::vector<Step> steps[2];
-    for (int u = 0; u < 2; ++u) {
-        int chunk = 0;
-        for (int t = 0; t < TILES; ++t) {
-            steps[u].push_back({0, 0});
-            for (int l = 0; l < sh.L - 1; ++l)
-                for (int ch = sh.nch - 1; ch >= 0; --ch, ++chunk) {
-                    steps[u].push_back({1, chunk});
-                    steps[u].push_back({2, 0});
-                    for (int kb = 2 * ch; kb < 2 * ch + 2; ++kb)
-                        if ((rd_mask[l] >> kb) & 1u) steps[u].push_back({3, kb});
-                    steps[u].push_back({4, ch});
-                }
-            for (int ch = sh.n_last - 1; ch >= 0; --ch, ++chunk) {
-                steps[u].push_back({1, chunk});
-                steps[u].push_back({2, 0});
-            }
-            for (int kb = 0; kb < 4; ++kb)
-                if ((rd_mask[sh.L - 1] >> kb) & 1u) steps[u].push_back({3, kb});
-        }
-    }
-    size_t ei[2] = {0, 0};
-    auto epi_step = [&](int u) -> bool {
-        if (ei[u] >= steps[u].size()) return false;
-        const Step& s = steps[u][ei[u]];
-        switch (s.kind) {
-            case 0:
-                for (int kb = 0; kb < sh.KB0; ++kb) complete(a_ready, a_ready_seen, 4 * u + kb);
-                break;
-            case 1:
-                if (d_full[u] < s.a + 1) return false;
-                d_full_seen[u] = s.a + 1;
-                break;
-            case 2: complete(d_empty, d_empty_seen, u); break;
-            case 3:
-                if (a_free[4 * u + s.a] <= a_free_seen[4 * u + s.a]) return false;
-                a_free_seen[4 * u + s.a]++;
-                break;
-            case 4:
-                complete(a_ready, a_ready_seen, 4 * u + 2 * s.a);
-                complete(a_ready, a_ready_seen, 4 * u + 2 * s.a + 1);
-                break;
-        }
-        ++ei[u];
-        return true;
-    };
-    for (;;) {
-        bool progress = false;
-        // policy: which agent runs greedily first (the others one step per round)
-        if (policy == 0) { while (mma_step()) progress = true; if (epi_step(0)) progress = true; if (epi_step(1)) progress = true; }
-        else if (policy == 1) { while (epi_step(0)) progress = true; while (epi_step(1)) progress = true; if (mma_step()) progress = true; }
-        else if (policy == 2) { while (epi_step(1)) progress = true; if (mma_step()) progress = true; if (epi_step(0)) progress = true; }
-        else { while (epi_step(0)) progress = true; if (mma_step()) progress = true; if (epi_step(1)) progress = true; }
-        if (!progress) break;
-    }
-    return ok && mi == TILES * n && ei[0] == steps[0].size() && ei[1] == steps[1].size();
-}
-
 }  // namespace
-
-std::atomic<int> g_dual{1};  // zk_set_dual_tiles
-
-static bool dual_dims_ok(const int* dims, int L, int univariate, int bins, int D, int C) {
-    if (!g_dual.load()) return false;
-    if (L < 2 || L > ZK_FUSED_MAX_LINEAR) return false;
-    const int H = dims[1];
-    if (H != 128 && H != 256) return false;
-    for (int i = 1; i < L; ++i)
-        if (dims[i] != H) return false;
-    if (D + C > 256 || dims[0] != D + C) return false;
-    if (univariate == ZK_UNI_RQS) return bins == 8 || bins == 16;
-    return univariate == ZK_UNI_AFFINE;
-}
-
-bool fused_dual_shape(const zk_mlp* m, int univariate, int bins, int D, int C) {
-    const TcPack* pk = (const TcPack*)m->tc;
-    if (!pk || m->gemm_mode == ZK_GEMM_FP32) return false;
-    if (!m->plain) return false;  // residual blocks: see fused_wide.cu
-    return dual_dims_ok(m->dims.data(), m->n_linear, univariate, bins, D, C);
-}
-
-// Pure host code: the issue schedule of one 512-row pair tile — per layer, chunks descending, the two
-// sub-tiles alternating chunk by chunk, K blocks descending inside a chunk.
-bool dual_build_schedule(const int* dims, int L, const std::vector<std::vector<uint8_t>>& Mk,
-                         const std::vector<std::vector<int>>& perm, int univariate, int bins, int D,
-                         std::vector<uint2>& items, uint32_t* rd_mask /*[8]*/) {
-    const int H = dims[1];
-    const int P = fused_p(univariate, bins), DPC = fused_dpc(univariate, bins);
-    DualShape sh;
-    sh.L = L; sh.nch = H / 128; sh.KB0 = pad64(dims[0]) / 64; sh.KBH = H / 64;
-    sh.n_last = (D + DPC - 1) / DPC;
-    std::vector<std::vector<uint32_t>> kbmask(L);
-    std::vector<std::vector<int>> kmax(L);  // [ch * 8 + kb]: last K column of the block any row of the chunk reads
-    for (int l = 0; l < L; ++l) {
-        const bool last = (l == L - 1);
-        const int K = dims[l], N = dims[l + 1];
-        const int nch = last ? sh.n_last : sh.nch;
-        kbmask[l].assign(nch, 0);
-        kmax[l].assign((size_t)nch * 8, 0);
-        for (int ch = 0; ch < nch; ++ch) {
-            const int n0 = last ? ch * DPC * P : ch * 128;
-            const int n1 = std::min(N, last ? n0 + DPC * P : n0 + 128);
-            uint32_t bits = 0;
-            for (int n = n0; n < n1; ++n) {
-                const int sn = (l < L - 1) ? perm[l][n] : n;
-                const uint8_t* mrow = &Mk[l][(size_t)sn * K];
-                for (int k = 0; k < K; ++k) {
-                    const int sk = (l > 0) ? perm[l - 1][k] : k;
-                    if (mrow[sk]) {
-                        bits |= 1u << (k / 64);
-                        kmax[l][(size_t)ch * 8 + k / 64] = std::max(kmax[l][(size_t)ch * 8 + k / 64], k % 64);
-                    }
-                }
-            }
-            if (bits == 0) bits = 1;
-            kbmask[l][ch] = bits;
-        }
-    }
-    items.clear();
-    for (int l = 0; l < 8; ++l) rd_mask[l] = 0u;
-    uint32_t written = (1u << sh.KB0) - 1u;  // per sub-tile: A blocks with a pending a_ready phase when the layer starts
-    for (int l = 0; l < L; ++l) {
-        const bool last = (l == L - 1);
-        const int nch = last ? sh.n_last : sh.nch;
-        const int KB = (l == 0) ? sh.KB0 : sh.KBH;
-        uint32_t rd = 0;
-        for (int ch = 0; ch < nch; ++ch) rd |= kbmask[l][ch] & ((1u << KB) - 1u);
-        rd_mask[l] = rd;
-        int last_reader[4];
-        for (int kb = 0; kb < 4; ++kb) last_reader[kb] = -1;
-        for (int ch = nch - 1; ch >= 0; --ch)
-            for (int kb = 0; kb < KB; ++kb)
-                if ((kbmask[l][ch] >> kb) & 1u) last_reader[kb] = ch;
-        uint32_t waited[2] = {0u, 0u};
-        size_t layer_first[2] = {(size_t)-1, (size_t)-1};
-        for (int ch = nch - 1; ch >= 0; --ch)
-            for (int u = 0; u < 2; ++u) {
-                const uint32_t kbm = kbmask[l][ch] & ((1u << KB) - 1u);
-                int lo = 0;
-                for (int kb = KB - 1; kb >= 0; --kb) if ((kbm >> kb) & 1u) lo = kb;
-                bool first = true;
-                for (int kb = KB - 1; kb >= 0; --kb) {
-                    if (!((kbm >> kb) & 1u)) continue;
-                    uint32_t it = (uint32_t)kb | ((uint32_t)u << 2) | (first ? DS_FIRST : 0u) | (kb == lo ? DS_LAST : 0u) | ((uint32_t)l << 16);
-                    if (!((waited[u] >> kb) & 1u)) { it |= DS_AWAIT; waited[u] |= 1u << kb; }
-                    if (last_reader[kb] == ch) it |= DS_AFREE;
-                    if (last) it |= DS_OUT;
-                    it |= (uint32_t)(3 - kmax[l][(size_t)ch * 8 + kb] / 16) << 20;  // trailing all-zero 16-column steps of the block are not issued
-                    if (layer_first[u] == (size_t)-1) layer_first[u] = items.size();
-                    items.push_back(make_uint2(it, (uint32_t)(last ? ch * DPC * P : ch * 128)));
-                    first = false;
-                }
-            }
-        for (int u = 0; u < 2; ++u) items[layer_first[u]].x |= ((written & ~rd) << (4 * u)) << 8;
-        written = last ? 0u : ((1u << sh.KBH) - 1u);
-    }
-    for (int policy = 0; policy < 4; ++policy)
-        if (!dual_dry_run(items, rd_mask, sh, policy)) return false;
-    return true;
-}
-
-// Host-only entry behind zk_debug_dual_schedule (tests): masks on the HOST, no CUDA call.
-int dual_schedule_host(int n_linear, const int* dims, const uint8_t* const* masks_host, int univariate, int bins, int D,
-                       int C, uint32_t* out_items, int max_items, uint32_t* out_rd_mask, int* out_perm) {
-    const int keep = g_dual.exchange(1);
-    const bool shape_ok = dual_dims_ok(dims, n_linear, univariate, bins, D, C);
-    g_dual.store(keep);
-    if (!shape_ok) return -1;
-    std::vector<std::vector<uint8_t>> Mk(n_linear);
-    for (int l = 0; l < n_linear; ++l) {
-        const size_t n = (size_t)dims[l + 1] * dims[l];
-        Mk[l].assign(n, 1);
-        if (masks_host && masks_host[l]) memcpy(Mk[l].data(), masks_host[l], n);
-    }
-    std::vector<std::vector<int>> perm;
-    fused_degree_perm(dims, n_linear, Mk, perm);
-    std::vector<uint2> items;
-    uint32_t rd[8];
-    if (!dual_build_schedule(dims, n_linear, Mk, perm, univariate, bins, D, items, rd)) return -2;
-    if ((int)items.size() > max_items) return -3;
-    for (size_t i = 0; i < items.size(); ++i) { out_items[2 * i] = items[i].x; out_items[2 * i + 1] = items[i].y; }
-    if (out_rd_mask) for (int l = 0; l < 8; ++l) out_rd_mask[l] = rd[l];
-    if (out_perm) {
-        size_t o = 0;
-        for (int l = 0; l < n_linear - 1; ++l)
-            for (int v : perm[l]) out_perm[o++] = v;
-    }
-    return (int)items.size();
-}
-
-zk_status fused_dual_prepare(zk_mlp* m, const uint8_t* const* mask_dev, int univariate, int bins, int D, int C) {
-    if (!fused_dual_shape(m, univariate, bins, D, C)) return ZK_OK;
-    TcPack* pk = (TcPack*)m->tc;
-    WidePack& wp = pk->dual;
-    wp.ready = false;
-    const int L = m->n_linear;
-    const int P = fused_p(univariate, bins), DPC = fused_dpc(univariate, bins);
-    const int N_LAST = (DPC * P + 15) & ~15;
-    FusedHostPrep hp;
-    ZK_TRY(fused_host_prepare(m, mask_dev, pk->fused, hp));
-    wp.maps.assign(L, CUtensorMap{});
-    for (int l = 0; l < L; ++l)
-        ZK_TRY(make_plane_map(&wp.maps[l], pk->fused.w[l], m->dims[l + 1], pk->layers[l].Kp, (l == L - 1) ? N_LAST / 2 : 64));
-    std::vector<uint2> items;
-    uint32_t rdm[8];
-    if (!dual_build_schedule(m->dims.data(), L, hp.Mk, hp.perm, univariate, bins, D, items, rdm)) return ZK_OK;
-    for (int l = 0; l < 8; ++l) wp.rd_mask[l] = (uint8_t)rdm[l];
-    {
-        double macs = 0;
-        for (const uint2& it : items) macs += 16.0 * (4 - (int)((it.x >> 20) & 3u)) * ((it.x & DS_OUT) ? N_LAST : 128);
-        wp.issued_macs_per_row = macs / 2 * pk->n_terms;  // the schedule covers two sub-tiles
-    }
-    cudaFree(wp.sched);
-    wp.sched = nullptr;
-    wp.n_items = (int)items.size();
-    if (cudaMalloc((void**)&wp.sched, items.size() * sizeof(uint2)) != cudaSuccess ||
-        cudaMemcpy(wp.sched, items.data(), items.size() * sizeof(uint2), cudaMemcpyHostToDevice) != cudaSuccess)
-        return fail(ZK_ENOMEM, "fused_dual_prepare: cudaMalloc failed");
-    wp.uni = univariate; wp.bins = bins; wp.D = D; wp.C = C;
-    wp.ready = true;
-    return ZK_OK;
-}
 
 zk_status launch_fused_dual(const zk_mlp* m, const FusedLayerArgs& a, cudaStream_t st) {
     const TcPack* pk = (const TcPack*)m->tc;
     ZK_REQUIRE(pk, "fused dual layer: no tensor-core pack");
     const WidePack& wp = pk->dual;
-    ZK_REQUIRE(wp.ready && wp.uni == a.univariate && wp.bins == a.bins && wp.D == a.D && wp.C == a.C && wp.sched,
+    ZK_REQUIRE(wp.built_for(a.univariate, a.bins, a.D, a.C) && wp.sched,
                "fused dual layer: the conditioner was not prepared for this bijector");
     ZK_REQUIRE(a.B < ((int64_t)1 << 31) - 4 * DM, "fused dual layer: batch too large for one launch");
     if (a.B == 0) return ZK_OK;
-    const int L = m->n_linear;
     DualParams p;
-    memset(&p, 0, sizeof(p));
-    const int DPC = fused_dpc(a.univariate, a.bins);
-    p.n_linear = L;
-    p.K0 = a.D + a.C;
-    p.KB0 = pk->layers[0].Kp / DK;
-    p.H = m->dims[1];
-    p.nch_hidden = p.H / 128;
-    p.D = a.D; p.C = a.C;
-    p.n_last_chunks = (a.D + DPC - 1) / DPC;
-    p.n_terms = pk->n_terms;
-    p.M = (int)a.B;
-    p.x = a.x; p.ldx = a.ldx; p.c = a.c; p.ldc = a.ldc;
-    p.y = a.y; p.ldy = a.ldy; p.ladj = a.ladj; p.accumulate = a.accumulate;
-    p.log_prob = a.log_prob; p.base_loc = a.base_loc; p.base_scale = a.base_scale;
-    p.bound = a.bound;
-    const float absL = fabsf(logf(a.slope));
-    p.aw = 2.f / absL;
-    p.ad = 1.f / absL;
-    p.dbg = g_timeline;
-    p.act = m->act;
-    p.sched = wp.sched;
-    p.n_items = wp.n_items;
-    const bool x_ok = (a.ldx % 4 == 0) && (a.D % 4 == 0) && (((uintptr_t)a.x) % 16 == 0);
-    const bool c_ok = (a.C == 0) || ((a.C % 4 == 0) && (((uintptr_t)a.c) % 16 == 0) && (a.ldc % 4 == 0));
-    p.in_vec = (x_ok && c_ok) ? 1 : 0;
+    pair_fill_params(p, m, wp, a);
     const uint32_t avail = D_SMEM_MAX - 1024u - D_ALO_BYTES - D_AUX_BYTES;
     p.n_wstages = (int)std::min<uint32_t>(D_MAX_WSTAGES, avail / D_WSTAGE);
     uint32_t bias_room = (avail - (uint32_t)p.n_wstages * D_WSTAGE) / 4u;
     int need_floats = a.log_prob ? ((3 * a.D + 3) & ~3) : 0;
-    for (int l = 0; l < L; ++l) need_floats += (m->dims[l + 1] + 3) & ~3;
+    for (int l = 0; l < m->n_linear; ++l) need_floats += (m->dims[l + 1] + 3) & ~3;
     while ((uint32_t)need_floats > bias_room && p.n_wstages > 3) { --p.n_wstages; bias_room += D_WSTAGE / 4u; }  // biases first
     ZK_REQUIRE(p.n_wstages >= 3, "fused dual layer: not enough shared memory for the weight ring");
-    int off = 0;
-    const int base_floats = a.log_prob ? ((3 * a.D + 3) & ~3) : 0;
-    ZK_REQUIRE((uint32_t)base_floats <= bias_room, "fused dual layer: no shared memory left for the base table");
-    bias_room -= (uint32_t)base_floats;
-    auto place = [&](int l) {
-        const int len = (m->dims[l + 1] + 3) & ~3;
-        p.bias[l] = pk->fused.bias[l];
-        p.bias_len[l] = m->dims[l + 1];
-        if ((uint32_t)(off + len) <= bias_room) { p.bias_off[l] = off; off += len; }
-        else p.bias_off[l] = -1;
-    };
-    place(L - 1);
-    for (int l = 0; l < L - 1; ++l) place(l);
-    for (int l = L; l < ZK_FUSED_MAX_LINEAR; ++l) { p.bias[l] = nullptr; p.bias_off[l] = -1; p.bias_len[l] = 0; }
-    for (int l = 0; l < L; ++l) { p.mapW[l] = wp.maps[l]; p.rd_mask[l] = wp.rd_mask[l]; }
-    p.base_off = off;
-    const size_t smem = 1024u + D_ALO_BYTES + (size_t)p.n_wstages * D_WSTAGE + D_AUX_BYTES + (size_t)(off + base_floats) * 4u;
-    if (g_watch_host == nullptr) {
-        uint32_t* h = nullptr;
-        if (cudaHostAlloc((void**)&h, 1024 * 4, cudaHostAllocMapped) == cudaSuccess) {
-            memset(h, 0, 1024 * 4);
-            g_watch_host = h;
-        } else {
-            cudaGetLastError();
-        }
-    }
-    p.watch = nullptr;
-    if (g_watch_host != nullptr) {
-        void* d = nullptr;
-        if (cudaHostGetDevicePointer(&d, g_watch_host, 0) == cudaSuccess) p.watch = (uint32_t*)d;
-        else cudaGetLastError();
-    }
+    uint32_t copy_floats = 0;
+    ZK_TRY(pair_place_biases(p, m, a, bias_room, "fused dual layer", copy_floats));
+    const size_t smem = 1024u + D_ALO_BYTES + (size_t)p.n_wstages * D_WSTAGE + D_AUX_BYTES + (size_t)copy_floats * 4u;
+    p.watch = pair_watch_device();
     const int64_t pairs = ceil_div(a.B, 4 * DM);
     const int grid = 2 * (int)std::min<int64_t>(pairs, sm_count() / 2);
     const bool rqs8 = a.univariate == ZK_UNI_RQS && a.bins == 8, rqs16 = a.univariate == ZK_UNI_RQS && a.bins == 16;

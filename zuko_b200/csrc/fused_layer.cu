@@ -637,27 +637,17 @@ static bool fused_narrow_shape(const zk_mlp* m, int univariate, int bins, int D,
     return univariate == ZK_UNI_AFFINE;
 }
 
-static bool wide_ready(const zk_mlp* m, int univariate, int bins, int D, int C) {
-    const TcPack* pk = (const TcPack*)m->tc;  // wide shapes: only once the issue schedule passed its dry run
-    return pk && fused_wide_shape(m, univariate, bins, D, C) && pk->wide.ready && pk->wide.uni == univariate &&
-           pk->wide.bins == bins && pk->wide.D == D && pk->wide.C == C;
-}
-
-static bool dual_ready(const zk_mlp* m, int univariate, int bins, int D, int C) {
-    const TcPack* pk = (const TcPack*)m->tc;
-    return pk && fused_dual_shape(m, univariate, bins, D, C) && pk->dual.ready && pk->dual.uni == univariate &&
-           pk->dual.bins == bins && pk->dual.D == D && pk->dual.C == C;
+int fused_layer_kind(const zk_mlp* m, int univariate, int bins, int D, int C) {
+    const TcPack* pk = (const TcPack*)m->tc;  // non-null once a shape test passed
+    // a pair kernel runs the layer once it takes the shape (routing knobs included) and its pack holds
+    // a schedule for this bijector
+    if (fused_dual_shape(m, univariate, bins, D, C) && pk->dual.built_for(univariate, bins, D, C)) return 3;
+    if (fused_wide_shape(m, univariate, bins, D, C) && pk->wide.built_for(univariate, bins, D, C)) return 2;
+    return fused_narrow_shape(m, univariate, bins, D, C) ? 1 : 0;
 }
 
 bool fused_layer_supported(const zk_mlp* m, int univariate, int bins, int D, int C) {
-    return fused_narrow_shape(m, univariate, bins, D, C) || wide_ready(m, univariate, bins, D, C) ||
-           dual_ready(m, univariate, bins, D, C);
-}
-
-int fused_layer_kind(const zk_mlp* m, int univariate, int bins, int D, int C) {
-    if (dual_ready(m, univariate, bins, D, C)) return 3;
-    if (wide_ready(m, univariate, bins, D, C)) return 2;
-    return fused_narrow_shape(m, univariate, bins, D, C) ? 1 : 0;
+    return fused_layer_kind(m, univariate, bins, D, C) != 0;
 }
 
 namespace {
@@ -677,41 +667,6 @@ __global__ void permute_bias_kernel(const float* b, int N, const int* perm, floa
     if (i < N) out[i] = b[perm ? perm[i] : i];
 }
 }  // namespace
-
-// Dependency degree of every hidden unit = number of network inputs it can see
-// (flows/autoregressive.py:121-124 + nn.py:270-293: units of a lower order class see fewer inputs);
-// sorting by degree makes the hidden -> hidden masks block lower-triangular.  Pure host code.
-void fused_degree_perm(const int* dims, int L, const std::vector<std::vector<uint8_t>>& Mk,
-                       std::vector<std::vector<int>>& perm) {
-    const int K0 = dims[0];
-    perm.assign(L - 1, {});  // perm[l][new] = old index of hidden layer l+1's units
-    // dependency sets as bit rows: dep[unit] = OR of the dep rows of the inputs it is connected to
-    const int W64 = (K0 + 63) / 64;
-    std::vector<uint64_t> prev, cur;
-    for (int l = 0; l < L - 1; ++l) {
-        const int K = dims[l], N = dims[l + 1];
-        cur.assign((size_t)N * W64, 0);
-        for (int n = 0; n < N; ++n) {
-            uint64_t* dn = &cur[(size_t)n * W64];
-            const uint8_t* mrow = &Mk[l][(size_t)n * K];
-            for (int k = 0; k < K; ++k) {
-                if (!mrow[k]) continue;
-                if (l == 0) dn[k >> 6] |= (uint64_t)1 << (k & 63);
-                else {
-                    const uint64_t* dk = &prev[(size_t)k * W64];
-                    for (int w = 0; w < W64; ++w) dn[w] |= dk[w];
-                }
-            }
-        }
-        std::vector<int> deg(N, 0);
-        for (int n = 0; n < N; ++n)
-            for (int w = 0; w < W64; ++w) deg[n] += __builtin_popcountll(cur[(size_t)n * W64 + w]);
-        perm[l].resize(N);
-        for (int n = 0; n < N; ++n) perm[l][n] = n;
-        std::stable_sort(perm[l].begin(), perm[l].end(), [&](int a, int b) { return deg[a] < deg[b]; });
-        prev.swap(cur);
-    }
-}
 
 // Masks to the host, hidden units sorted by dependency degree, permuted bf16 hi / lo planes and
 // biases on the device (shared by the narrow and the wide fused kernel).
@@ -787,16 +742,16 @@ zk_status fused_refresh(zk_mlp* m, cudaStream_t st) {
 }
 
 zk_status fused_layer_prepare(zk_mlp* m, const uint8_t* const* mask_dev, int univariate, int bins, int D, int C) {
+    TcPack* pk = (TcPack*)m->tc;
     if (fused_dual_shape(m, univariate, bins, D, C)) {  // two sub-tiles in flight (hidden width 128 / 256)
-        ZK_TRY(fused_dual_prepare(m, mask_dev, univariate, bins, D, C));
-        if (dual_ready(m, univariate, bins, D, C)) return ZK_OK;
+        ZK_TRY(fused_pair_prepare(m, mask_dev, univariate, bins, D, C, pk->dual, 2));
+        if (pk->dual.ready) return ZK_OK;
     }
     if (fused_wide_shape(m, univariate, bins, D, C)) {  // CTA-pair kernel; hidden width 256 may fall back to the narrow one
-        ZK_TRY(fused_wide_prepare(m, mask_dev, univariate, bins, D, C));
-        if (wide_ready(m, univariate, bins, D, C)) return ZK_OK;
+        ZK_TRY(fused_pair_prepare(m, mask_dev, univariate, bins, D, C, pk->wide, 1));
+        if (pk->wide.ready) return ZK_OK;
     }
     if (!fused_narrow_shape(m, univariate, bins, D, C)) return ZK_OK;
-    TcPack* pk = (TcPack*)m->tc;
     FusedPack& f = pk->fused;
     const int L = m->n_linear;
     const int H = m->dims[1];
@@ -805,40 +760,19 @@ zk_status fused_layer_prepare(zk_mlp* m, const uint8_t* const* mask_dev, int uni
     const int DPC = fused_dpc(univariate, bins);
     FusedHostPrep hp;
     ZK_TRY(fused_host_prepare(m, mask_dev, f, hp));
-    const std::vector<std::vector<uint8_t>>& Mk = hp.Mk;
-    const std::vector<std::vector<int>>& perm = hp.perm;
     f.map64.clear();
     f.map64.resize(L);
     for (int l = 0; l < L; ++l) ZK_TRY(make_plane_map(&f.map64[l], f.w[l], m->dims[l + 1], pk->layers[l].Kp, 64));
-    // ---- which (chunk, K block) tiles of the permuted masked matrices are non-zero ----
+    const FusedTileMap tm = fused_tile_map(m->dims.data(), L, hp.Mk, hp.perm, CW, univariate, bins, D);
     memset(f.kbmask, 0, sizeof(f.kbmask));
-    for (int l = 0; l < L; ++l) {
-        const bool last = (l == L - 1);
-        const int K = m->dims[l], N = m->dims[l + 1];
-        const int nch = last ? (D + DPC - 1) / DPC : H / CW;
-        const int KB = pk->layers[l].Kp / 64;
-        for (int ch = 0; ch < nch && ch < 128; ++ch) {
-            const int n0 = last ? ch * DPC * P : ch * CW;
-            const int n1 = std::min(N, last ? n0 + DPC * P : n0 + CW);
-            uint8_t bits = 0;
-            for (int n = n0; n < n1; ++n) {
-                const int sn = (l < L - 1) ? perm[l][n] : n;
-                for (int k = 0; k < K; ++k) {
-                    const int sk = (l > 0) ? perm[l - 1][k] : k;
-                    if (Mk[l][(size_t)sn * K + sk]) bits |= (uint8_t)(1u << (k / 64));
-                }
-            }
-            if (bits == 0) bits = 1;  // the accumulator still has to be defined (bias-only outputs)
-            (void)KB;
-            f.kbmask[l][ch] = bits;
-        }
-    }
+    for (int l = 0; l < L; ++l)
+        for (size_t ch = 0; ch < tm.kbmask[l].size() && ch < 128; ++ch) f.kbmask[l][ch] = (uint8_t)tm.kbmask[l][ch];
     // ---- MMA issue schedule of one tile: one entry per non-zero (layer, chunk, K block) tile, in the
     //      order the W producer streams them (bit layout: see the MMA issuer in the kernel) ----
     std::vector<uint32_t> items;
     for (int l = 0; l < L; ++l) {
         const bool last = (l == L - 1);
-        const int nch = std::min(128, last ? (D + DPC - 1) / DPC : H / CW);
+        const int nch = std::min(128, (int)tm.kbmask[l].size());
         const int KB = (l == 0) ? pk->layers[0].Kp / 64 : H / 64;
         int last_reader[F_MAXKB];
         for (int kb = 0; kb < F_MAXKB; ++kb) last_reader[kb] = -1;
@@ -887,8 +821,9 @@ zk_status fused_layer_prepare(zk_mlp* m, const uint8_t* const* mask_dev, int uni
 
 zk_status launch_fused_layer(const zk_mlp* m, const FusedLayerArgs& a, cudaStream_t st) {
     const TcPack* pk = (const TcPack*)m->tc;
-    if (dual_ready(m, a.univariate, a.bins, a.D, a.C)) return launch_fused_dual(m, a, st);
-    if (wide_ready(m, a.univariate, a.bins, a.D, a.C)) return launch_fused_wide(m, a, st);
+    const int kind = fused_layer_kind(m, a.univariate, a.bins, a.D, a.C);
+    if (kind == 3) return launch_fused_dual(m, a, st);
+    if (kind == 2) return launch_fused_wide(m, a, st);
     ZK_REQUIRE(pk && fused_narrow_shape(m, a.univariate, a.bins, a.D, a.C), "fused layer: unsupported shape");
     ZK_REQUIRE(a.B < ((int64_t)1 << 31) - FM, "fused layer: batch too large for one launch");
     if (a.B == 0) return ZK_OK;

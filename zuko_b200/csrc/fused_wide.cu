@@ -21,7 +21,7 @@
 //     nobody reads the top K blocks again and its own outputs (the next layer's top K blocks) can
 //     overwrite them, and so on down.  The next layer starts with the K blocks that were written
 //     first, so the tensor pipe does not drain at layer boundaries.  The order and every barrier
-//     obligation are a table built (and dry-run for deadlocks) on the host: fused_wide_prepare.
+//     obligation are a table built (and dry-run for deadlocks) on the host: fused_plan.cu.
 //
 // Tensor memory (512 columns x 128 lanes, lane = sample row of this CTA's half tile):
 //   [  0,256)  A hi : bf16 pairs, K element k in column k/2                     (K <= 512)
@@ -44,18 +44,13 @@
 //   warps 4-19  epilogue (both CTAs; their "buffer drained" / "A block written" arrivals go to the
 //               leader's barriers through the cluster shared-memory window)
 
-#include <string.h>
-
 #include <algorithm>
-#include <atomic>
 
 #include "activations.cuh"
 #include "fused_common.cuh"
 #include "pair_common.cuh"
 
 namespace zk {
-
-uint32_t* g_watch_host = nullptr;  // mapped pinned host memory the kernel's watchdog reports into
 
 namespace {
 
@@ -75,15 +70,8 @@ constexpr uint32_t W_BAR_SLOTS = 40;                          // 36 mbarriers + 
 constexpr uint32_t W_AUX_BYTES = W_BAR_SLOTS * 8 + 2 * 3 * WM * 4;  // + ladj partials [2][3][128]
 constexpr uint32_t W_SMEM_MAX = 232448;                       // 227 KB per CTA on sm_100
 constexpr uint32_t TMW_D = 256;                               // first accumulator column
-constexpr int W_WATCH_WORDS = 1024;
 
-// schedule entry (uint2): x = flags, y = first weight row of the chunk
-//   x [2:0] K block | [3] first K block of its chunk | [4] last K block of its chunk |
-//     [5] first read of A block kb in this layer (wait a_ready[kb]) | [6] last read of A block kb in this
-//     layer (commit a_free[kb]) | [7] output layer | [15:8] a_ready phases the layer consumes without
-//     reading (on the layer's first entry) | [18:16] layer |
-//     [21:20] trailing 16-column MMA steps of the K block that are all-zero for this chunk (not issued)
-constexpr uint32_t WS_FIRST = 8u, WS_LAST = 16u, WS_AWAIT = 32u, WS_AFREE = 64u, WS_OUT = 128u;
+// schedule entries: pair_common.cuh (S = 1: bits [2:0] are the K block)
 
 struct WideParams {
     CUtensorMap mapW[ZK_FUSED_MAX_LINEAR];
@@ -559,362 +547,31 @@ zk_status launch_wide_t(const WideParams& p, bool fast, int grid, size_t smem, c
     return go(fused_wide_kernel<UNI, KT, false, false, false>);
 }
 
-// ---------------------------------------------------------------------------
-// host: schedule + dry run
-// ---------------------------------------------------------------------------
-struct WideShape {
-    int L, H, nch, KB0, KBH, n_last, DPC, P;
-};
-
-// One pair tile's work as the kernel walks it, two tiles back to back, under the barrier protocol of
-// the kernel: a schedule that can deadlock, or lets a barrier run two phases ahead of its waiter
-// (parity aliasing), is rejected and the layer stays on the per-layer path.
-bool wide_dry_run(const std::vector<uint2>& items, const uint32_t* rd_mask, const WideShape& sh, bool epilogue_first) {
-    const int n = (int)items.size();
-    const int TILES = 3;
-    // completed phases
-    int d_full[2] = {0, 0}, d_empty[2] = {0, 0}, a_ready[8] = {0}, a_free[8] = {0};
-    // phases seen by the waiter
-    int d_full_seen[2] = {0, 0}, d_empty_seen[2] = {0, 0}, a_ready_seen[8] = {0}, a_free_seen[8] = {0};
-    bool ok = true;
-    auto complete = [&](int* done, const int* seen, int idx) {
-        if (done[idx] != seen[idx]) ok = false;  // the waiter has not consumed the previous phase yet
-        done[idx]++;
-    };
-    // ---- MMA side (scout + issuer) ----
-    int mi = 0;
-    uint32_t mc = 0;
-    auto mma_step = [&]() -> bool {
-        if (mi >= TILES * n) return false;
-        const uint32_t it = items[mi % n].x;
-        uint32_t c = mc;
-        if (mi > 0 && (it & WS_FIRST)) c = mc + 1;
-        const int buf = (int)(c & 1u);
-        if (it & WS_FIRST) {
-            // the k-th use of a buffer needs k drains (k = c >> 1)
-            if (d_empty[buf] < (int)(c >> 1)) return false;
-        }
-        for (int k2 = 0; k2 < 8; ++k2)
-            if ((it >> (8 + k2)) & 1u)
-                if (a_ready[k2] <= a_ready_seen[k2]) return false;
-        if (it & WS_AWAIT) {
-            const int kb = (int)(it & 7u);
-            if (a_ready[kb] <= a_ready_seen[kb]) return false;
-        }
-        // all prerequisites met: consume and issue (MMAs complete in order, at once)
-        if (it & WS_FIRST) d_empty_seen[buf] = (int)(c >> 1);
-        for (int k2 = 0; k2 < 8; ++k2)
-            if ((it >> (8 + k2)) & 1u) a_ready_seen[k2]++;
-        if (it & WS_AWAIT) a_ready_seen[it & 7u]++;
-        if (it & WS_AFREE) complete(a_free, a_free_seen, (int)(it & 7u));
-        if (it & WS_LAST) complete(d_full, d_full_seen, buf);
-        mc = c;
-        ++mi;
-        return true;
-    };
-    // ---- epilogue side: a flat list of steps per tile ----
-    struct Step { int kind, a, b; };  // 0 stage, 1 wait d_full(chunk), 2 drain(buf), 3 wait a_free(kb), 4 write(ch)
-    std::vector<Step> steps;
-    {
-        for (int t = 0; t < TILES; ++t) {
-            int chunk_base = t * ((sh.L - 1) * sh.nch + sh.n_last);
-            int chunk = chunk_base;
-            steps.push_back({0, 0, 0});
-            for (int l = 0; l < sh.L - 1; ++l)
-                for (int ch = sh.nch - 1; ch >= 0; --ch, ++chunk) {
-                    steps.push_back({1, chunk, 0});
-                    steps.push_back({2, chunk & 1, 0});
-                    for (int kb = 2 * ch; kb < 2 * ch + 2; ++kb)
-                        if ((rd_mask[l] >> kb) & 1u) steps.push_back({3, kb, 0});
-                    steps.push_back({4, ch, 0});
-                }
-            for (int ch = sh.n_last - 1; ch >= 0; --ch, ++chunk) {
-                steps.push_back({1, chunk, 0});
-                steps.push_back({2, chunk & 1, 0});
-            }
-            for (int kb = 0; kb < 8; ++kb)
-                if ((rd_mask[sh.L - 1] >> kb) & 1u) steps.push_back({3, kb, 0});
-        }
-    }
-    size_t ei = 0;
-    auto epi_step = [&]() -> bool {
-        if (ei >= steps.size()) return false;
-        const Step& s = steps[ei];
-        switch (s.kind) {
-            case 0:
-                for (int kb = 0; kb < sh.KB0; ++kb) complete(a_ready, a_ready_seen, kb);
-                break;
-            case 1: {
-                const int buf = s.a & 1, need = (s.a >> 1) + 1;
-                if (d_full[buf] < need) return false;
-                d_full_seen[buf] = need;
-                break;
-            }
-            case 2: complete(d_empty, d_empty_seen, s.a); break;
-            case 3:
-                if (a_free[s.a] <= a_free_seen[s.a]) return false;
-                a_free_seen[s.a]++;
-                break;
-            case 4:
-                complete(a_ready, a_ready_seen, 2 * s.a);
-                complete(a_ready, a_ready_seen, 2 * s.a + 1);
-                break;
-        }
-        ++ei;
-        return true;
-    };
-    // d_empty bookkeeping: the scout's parity wait for the k-th use passes on phase k - 1 ... the
-    // "seen" counter above is set when it passes, so `complete` flags a drain that outruns it by two.
-    for (;;) {
-        bool progress = false;
-        if (epilogue_first) {
-            while (epi_step()) progress = true;
-            if (mma_step()) progress = true;
-        } else {
-            while (mma_step()) progress = true;
-            if (epi_step()) progress = true;
-        }
-        if (!progress) break;
-    }
-    return ok && mi == TILES * n && ei == steps.size();
-}
-
 }  // namespace
-
-std::atomic<int> g_wide_min_h{256};  // smallest hidden width routed to this kernel (zk_set_wide_min_hidden)
-
-static bool wide_dims_ok(const int* dims, int L, int univariate, int bins, int D, int C) {
-    if (L < 2 || L > ZK_FUSED_MAX_LINEAR) return false;
-    const int H = dims[1];
-    if (H % 128 != 0 || H < std::max(256, g_wide_min_h.load()) || H > 512) return false;
-    for (int i = 1; i < L; ++i)
-        if (dims[i] != H) return false;
-    if (D + C > 512 || dims[0] != D + C) return false;
-    if (univariate == ZK_UNI_RQS) return bins == 8 || bins == 16;
-    return univariate == ZK_UNI_AFFINE;
-}
-
-bool fused_wide_shape(const zk_mlp* m, int univariate, int bins, int D, int C) {
-    const TcPack* pk = (const TcPack*)m->tc;
-    if (!pk || m->gemm_mode == ZK_GEMM_FP32) return false;
-    if (!m->plain) return false;  // residual blocks need the input of two layers back, which the in-place update overwrote
-    return wide_dims_ok(m->dims.data(), m->n_linear, univariate, bins, D, C);
-}
-
-// Pure host code: the issue schedule of one pair tile for a conditioner with layer widths `dims`
-// (n_linear + 1 entries), host masks Mk and degree permutations perm.  Returns false when the
-// protocol dry run rejects the schedule (the layer then stays on the per-layer path).
-bool wide_build_schedule(const int* dims, int L, const std::vector<std::vector<uint8_t>>& Mk,
-                         const std::vector<std::vector<int>>& perm, int univariate, int bins, int D,
-                         std::vector<uint2>& items, uint32_t* rd_mask /*[8]*/) {
-    const int H = dims[1];
-    const int P = fused_p(univariate, bins), DPC = fused_dpc(univariate, bins);
-    WideShape sh;
-    sh.L = L; sh.H = H; sh.nch = H / 128; sh.KB0 = pad64(dims[0]) / 64; sh.KBH = H / 64;
-    sh.n_last = (D + DPC - 1) / DPC; sh.DPC = DPC; sh.P = P;
-    // ---- which (chunk, K block) tiles of the permuted masked matrices are non-zero ----
-    std::vector<std::vector<uint32_t>> kbmask(L);
-    std::vector<std::vector<int>> kmax(L);  // [ch * 8 + kb]: last K column of the block any row of the chunk reads
-    for (int l = 0; l < L; ++l) {
-        const bool last = (l == L - 1);
-        const int K = dims[l], N = dims[l + 1];
-        const int nch = last ? sh.n_last : sh.nch;
-        kbmask[l].assign(nch, 0);
-        kmax[l].assign((size_t)nch * 8, 0);
-        for (int ch = 0; ch < nch; ++ch) {
-            const int n0 = last ? ch * DPC * P : ch * 128;
-            const int n1 = std::min(N, last ? n0 + DPC * P : n0 + 128);
-            uint32_t bits = 0;
-            for (int n = n0; n < n1; ++n) {
-                const int sn = (l < L - 1) ? perm[l][n] : n;
-                const uint8_t* mrow = &Mk[l][(size_t)sn * K];
-                for (int k = 0; k < K; ++k) {
-                    const int sk = (l > 0) ? perm[l - 1][k] : k;
-                    if (mrow[sk]) {
-                        bits |= 1u << (k / 64);
-                        kmax[l][(size_t)ch * 8 + k / 64] = std::max(kmax[l][(size_t)ch * 8 + k / 64], k % 64);
-                    }
-                }
-            }
-            if (bits == 0) bits = 1;  // the accumulator still has to be defined (bias-only outputs)
-            kbmask[l][ch] = bits;
-        }
-    }
-    // ---- issue schedule: chunks and K blocks in DESCENDING order (see the header) ----
-    items.clear();
-    for (int l = 0; l < 8; ++l) rd_mask[l] = 0u;
-    uint32_t written = (1u << sh.KB0) - 1u;  // A blocks with a pending a_ready phase when the layer starts
-    for (int l = 0; l < L; ++l) {
-        const bool last = (l == L - 1);
-        const int nch = last ? sh.n_last : sh.nch;
-        const int KB = (l == 0) ? sh.KB0 : sh.KBH;
-        uint32_t rd = 0;
-        for (int ch = 0; ch < nch; ++ch) rd |= kbmask[l][ch] & ((1u << KB) - 1u);
-        rd_mask[l] = rd;
-        int last_reader[8];
-        for (int kb = 0; kb < 8; ++kb) last_reader[kb] = -1;
-        for (int ch = nch - 1; ch >= 0; --ch)  // issue order: the last reader is the lowest chunk
-            for (int kb = 0; kb < KB; ++kb)
-                if ((kbmask[l][ch] >> kb) & 1u) last_reader[kb] = ch;
-        uint32_t waited = 0;
-        const size_t layer_first = items.size();
-        for (int ch = nch - 1; ch >= 0; --ch) {
-            const uint32_t kbm = kbmask[l][ch] & ((1u << KB) - 1u);
-            int lo = 0;
-            for (int kb = KB - 1; kb >= 0; --kb) if ((kbm >> kb) & 1u) lo = kb;
-            bool first = true;
-            for (int kb = KB - 1; kb >= 0; --kb) {
-                if (!((kbm >> kb) & 1u)) continue;
-                uint32_t it = (uint32_t)kb | (first ? WS_FIRST : 0u) | (kb == lo ? WS_LAST : 0u) | ((uint32_t)l << 16);
-                if (!((waited >> kb) & 1u)) { it |= WS_AWAIT; waited |= 1u << kb; }
-                if (last_reader[kb] == ch) it |= WS_AFREE;
-                if (last) it |= WS_OUT;
-                it |= (uint32_t)(3 - kmax[l][(size_t)ch * 8 + kb] / 16) << 20;  // trailing all-zero 16-column steps of the block are not issued
-                items.push_back(make_uint2(it, (uint32_t)(last ? ch * DPC * P : ch * 128)));
-                first = false;
-            }
-        }
-        items[layer_first].x |= (written & ~rd) << 8;  // written for this layer but never read by it
-        written = last ? 0u : ((1u << sh.KBH) - 1u);
-    }
-    return wide_dry_run(items, rd_mask, sh, false) && wide_dry_run(items, rd_mask, sh, true);
-}
-
-// Host-only entry behind zk_debug_wide_schedule (tests): masks on the HOST, no CUDA call.
-int wide_schedule_host(int n_linear, const int* dims, const uint8_t* const* masks_host, int univariate, int bins, int D,
-                       int C, uint32_t* out_items, int max_items, uint32_t* out_rd_mask, int* out_perm) {
-    if (!wide_dims_ok(dims, n_linear, univariate, bins, D, C)) return -1;
-    std::vector<std::vector<uint8_t>> Mk(n_linear);
-    for (int l = 0; l < n_linear; ++l) {
-        const size_t n = (size_t)dims[l + 1] * dims[l];
-        Mk[l].assign(n, 1);
-        if (masks_host && masks_host[l]) memcpy(Mk[l].data(), masks_host[l], n);
-    }
-    std::vector<std::vector<int>> perm;
-    fused_degree_perm(dims, n_linear, Mk, perm);
-    std::vector<uint2> items;
-    uint32_t rd[8];
-    if (!wide_build_schedule(dims, n_linear, Mk, perm, univariate, bins, D, items, rd)) return -2;
-    if ((int)items.size() > max_items) return -3;
-    for (size_t i = 0; i < items.size(); ++i) { out_items[2 * i] = items[i].x; out_items[2 * i + 1] = items[i].y; }
-    if (out_rd_mask) for (int l = 0; l < 8; ++l) out_rd_mask[l] = rd[l];
-    if (out_perm) {
-        size_t o = 0;
-        for (int l = 0; l < n_linear - 1; ++l)
-            for (int v : perm[l]) out_perm[o++] = v;
-    }
-    return (int)items.size();
-}
-
-zk_status fused_wide_prepare(zk_mlp* m, const uint8_t* const* mask_dev, int univariate, int bins, int D, int C) {
-    if (!fused_wide_shape(m, univariate, bins, D, C)) return ZK_OK;
-    TcPack* pk = (TcPack*)m->tc;
-    WidePack& wp = pk->wide;
-    wp.ready = false;
-    const int L = m->n_linear;
-    const int P = fused_p(univariate, bins), DPC = fused_dpc(univariate, bins);
-    const int N_LAST = (DPC * P + 15) & ~15;
-    FusedHostPrep hp;
-    ZK_TRY(fused_host_prepare(m, mask_dev, pk->fused, hp));
-    wp.maps.assign(L, CUtensorMap{});
-    for (int l = 0; l < L; ++l)
-        ZK_TRY(make_plane_map(&wp.maps[l], pk->fused.w[l], m->dims[l + 1], pk->layers[l].Kp, (l == L - 1) ? N_LAST / 2 : 64));
-    std::vector<uint2> items;
-    uint32_t rdm[8];
-    if (!wide_build_schedule(m->dims.data(), L, hp.Mk, hp.perm, univariate, bins, D, items, rdm)) return ZK_OK;  // per-layer path
-    for (int l = 0; l < 8; ++l) wp.rd_mask[l] = (uint8_t)rdm[l];
-    {
-        double macs = 0;
-        for (const uint2& it : items) macs += 16.0 * (4 - (int)((it.x >> 20) & 3u)) * ((it.x & WS_OUT) ? N_LAST : 128);
-        wp.issued_macs_per_row = macs * pk->n_terms;
-    }
-    cudaFree(wp.sched);
-    wp.sched = nullptr;
-    wp.n_items = (int)items.size();
-    if (cudaMalloc((void**)&wp.sched, items.size() * sizeof(uint2)) != cudaSuccess ||
-        cudaMemcpy(wp.sched, items.data(), items.size() * sizeof(uint2), cudaMemcpyHostToDevice) != cudaSuccess)
-        return fail(ZK_ENOMEM, "fused_wide_prepare: cudaMalloc failed");
-    wp.uni = univariate; wp.bins = bins; wp.D = D; wp.C = C;
-    wp.ready = true;
-    return ZK_OK;
-}
 
 zk_status launch_fused_wide(const zk_mlp* m, const FusedLayerArgs& a, cudaStream_t st) {
     const TcPack* pk = (const TcPack*)m->tc;
     ZK_REQUIRE(pk && fused_wide_shape(m, a.univariate, a.bins, a.D, a.C), "fused wide layer: unsupported shape");
     const WidePack& wp = pk->wide;
-    ZK_REQUIRE(wp.ready && wp.uni == a.univariate && wp.bins == a.bins && wp.D == a.D && wp.C == a.C && wp.sched,
+    ZK_REQUIRE(wp.built_for(a.univariate, a.bins, a.D, a.C) && wp.sched,
                "fused wide layer: the conditioner was not prepared for this bijector");
     ZK_REQUIRE(a.B < ((int64_t)1 << 31) - 2 * WM, "fused wide layer: batch too large for one launch");
     if (a.B == 0) return ZK_OK;
-    const int L = m->n_linear;
     WideParams p;
-    memset(&p, 0, sizeof(p));
-    const int DPC = fused_dpc(a.univariate, a.bins);
-    p.n_linear = L;
-    p.K0 = a.D + a.C;
-    p.KB0 = pk->layers[0].Kp / WK;
-    p.H = m->dims[1];
-    p.nch_hidden = p.H / 128;
-    p.D = a.D; p.C = a.C;
-    p.n_last_chunks = (a.D + DPC - 1) / DPC;
-    p.n_terms = pk->n_terms;
-    p.M = (int)a.B;
-    p.x = a.x; p.ldx = a.ldx; p.c = a.c; p.ldc = a.ldc;
-    p.y = a.y; p.ldy = a.ldy; p.ladj = a.ladj; p.accumulate = a.accumulate;
-    p.log_prob = a.log_prob; p.base_loc = a.base_loc; p.base_scale = a.base_scale;
-    p.bound = a.bound;
-    const float absL = fabsf(logf(a.slope));
-    p.aw = 2.f / absL;
-    p.ad = 1.f / absL;
-    p.dbg = g_timeline;
-    p.sched = wp.sched;
-    p.n_items = wp.n_items;
-    const bool x_ok = (a.ldx % 4 == 0) && (a.D % 4 == 0) && (((uintptr_t)a.x) % 16 == 0);
-    const bool c_ok = (a.C == 0) || ((a.C % 4 == 0) && (((uintptr_t)a.c) % 16 == 0) && (a.ldc % 4 == 0));
-    p.in_vec = (x_ok && c_ok) ? 1 : 0;
+    pair_fill_params(p, m, wp, a);
     // shared memory: A lo + aux are fixed; the weight ring gets what is left after the bias copy of
-    // the OUTPUT layer (47 reads per dim and thread) and as many hidden-layer biases as still fit
+    // the OUTPUT layer and as many hidden-layer biases as still fit
     p.alo_blocks = std::max(p.KB0, p.H / WK);
-    p.act = m->act;
     const uint32_t alo_bytes = (uint32_t)p.alo_blocks * W_APLANE;
     const uint32_t avail = W_SMEM_MAX - 1024u - alo_bytes - W_AUX_BYTES;
     p.n_wstages = (int)std::min<uint32_t>(W_MAX_WSTAGES, avail / W_WSTAGE);
     uint32_t bias_room = (avail - (uint32_t)p.n_wstages * W_WSTAGE) / 4u;  // floats
     if (bias_room < 64u && p.n_wstages > 4) { --p.n_wstages; bias_room += W_WSTAGE / 4u; }
     ZK_REQUIRE(p.n_wstages >= 3, "fused wide layer: not enough shared memory for the weight ring");
-    int off = 0;
-    const int base_floats = a.log_prob ? ((3 * a.D + 3) & ~3) : 0;
-    ZK_REQUIRE((uint32_t)base_floats <= bias_room, "fused wide layer: no shared memory left for the base table");
-    bias_room -= (uint32_t)base_floats;
-    auto place = [&](int l) {
-        const int len = (m->dims[l + 1] + 3) & ~3;  // keep every layer's bias 16-byte aligned
-        p.bias[l] = pk->fused.bias[l];
-        p.bias_len[l] = m->dims[l + 1];
-        if ((uint32_t)(off + len) <= bias_room) { p.bias_off[l] = off; off += len; }
-        else p.bias_off[l] = -1;
-    };
-    place(L - 1);
-    for (int l = 0; l < L - 1; ++l) place(l);
-    for (int l = L; l < ZK_FUSED_MAX_LINEAR; ++l) { p.bias[l] = nullptr; p.bias_off[l] = -1; p.bias_len[l] = 0; }
-    for (int l = 0; l < L; ++l) { p.mapW[l] = wp.maps[l]; p.rd_mask[l] = wp.rd_mask[l]; }
-    p.base_off = off;
-    const size_t smem = 1024u + alo_bytes + (size_t)p.n_wstages * W_WSTAGE + W_AUX_BYTES + (size_t)(off + base_floats) * 4u;
-    if (g_watch_host == nullptr) {
-        uint32_t* h = nullptr;
-        if (cudaHostAlloc((void**)&h, W_WATCH_WORDS * 4, cudaHostAllocMapped) == cudaSuccess) {
-            memset(h, 0, W_WATCH_WORDS * 4);
-            g_watch_host = h;
-        } else {
-            cudaGetLastError();
-        }
-    }
-    p.watch = nullptr;
-    if (g_watch_host != nullptr) {
-        void* d = nullptr;
-        if (cudaHostGetDevicePointer(&d, g_watch_host, 0) == cudaSuccess) p.watch = (uint32_t*)d;
-        else cudaGetLastError();
-    }
+    uint32_t copy_floats = 0;
+    ZK_TRY(pair_place_biases(p, m, a, bias_room, "fused wide layer", copy_floats));
+    const size_t smem = 1024u + alo_bytes + (size_t)p.n_wstages * W_WSTAGE + W_AUX_BYTES + (size_t)copy_floats * 4u;
+    p.watch = pair_watch_device();
     const int64_t pairs = ceil_div(a.B, 2 * WM);
     const int grid = 2 * (int)std::min<int64_t>(pairs, sm_count() / 2);
     const bool rqs8 = a.univariate == ZK_UNI_RQS && a.bins == 8, rqs16 = a.univariate == ZK_UNI_RQS && a.bins == 16;

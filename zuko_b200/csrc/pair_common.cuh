@@ -1,7 +1,11 @@
-// zuko_b200 — what the CTA-pair fused kernels (fused_wide.cu, fused_dual.cu) share: the cta_group::2
-// forms of the tcgen05 / TMA / mbarrier instructions, the bounded waits with their watchdog report,
-// and the store of an A-operand lo plane fragment into its swizzled shared-memory layout.
+// zuko_b200 — what the CTA-pair fused kernels (fused_wide.cu, fused_dual.cu) share: the layout of their
+// schedule entries, the cta_group::2 forms of the tcgen05 / TMA / mbarrier instructions, the bounded
+// waits with their watchdog report, the store of an A-operand lo plane fragment into its swizzled
+// shared-memory layout, and the host code that fills their launch parameters.  The schedule itself is
+// built and dry-run in fused_plan.cu.
 #pragma once
+
+#include <string.h>
 
 #include "fused_common.cuh"
 
@@ -9,6 +13,16 @@ namespace zk {
 
 constexpr uint32_t W_APLANE = 128 * 64 * 2;       // 16 KB: one K block (128 rows x 64 bf16) of the A lo plane
 constexpr long long W_WD_CYCLES = 4000000000ll;   // watchdog: ~2 s of SM clock
+
+// schedule entry (uint2) of a kernel with S sub-tiles per CTA (fused_wide.cu: 1, fused_dual.cu: 2):
+// x = flags, y = first weight row of the chunk
+//   x [2:0] A block u * (8 / S) + kb of sub-tile u (S = 2: bit 2 is the sub-tile, kb < 4) |
+//     [3] first K block of its chunk | [4] last K block of its chunk |
+//     [5] first read of the A block in this layer (wait a_ready) | [6] last read of the A block in this
+//     layer (commit a_free) | [7] output layer | [15:8] a_ready phases (by A block) the layer consumes
+//     without reading (on the sub-tile's first entry of the layer) | [18:16] layer |
+//     [21:20] trailing 16-column MMA steps of the K block that are all-zero for this chunk (not issued)
+constexpr uint32_t WS_FIRST = 8u, WS_LAST = 16u, WS_AWAIT = 32u, WS_AFREE = 64u, WS_OUT = 128u;
 
 // ---------------------------------------------------------------------------
 // PTX: the cta_group::2 forms
@@ -128,6 +142,70 @@ __device__ __forceinline__ void st_alo32(uint8_t* sAlo, int kb, int r, int half,
         const int j = half * 4 + u;
         *reinterpret_cast<uint4*>(row + (((j ^ (r & 7)) & 7) << 4)) = make_uint4(pl[4 * u], pl[4 * u + 1], pl[4 * u + 2], pl[4 * u + 3]);
     }
+}
+
+// ---------------------------------------------------------------------------
+// host: launch parameters both kernels fill alike (WideParams and DualParams share these field names)
+// ---------------------------------------------------------------------------
+uint32_t* pair_watch_device();  // the watchdog buffer (allocated on first use) as the device sees it, or null
+
+// Zeroes `p`, then fills in the layer's arguments, its shapes and the schedule and tensor maps of `wp`.
+template <class Params>
+void pair_fill_params(Params& p, const zk_mlp* m, const WidePack& wp, const FusedLayerArgs& a) {
+    const TcPack* pk = (const TcPack*)m->tc;
+    const int DPC = fused_dpc(a.univariate, a.bins);
+    memset(&p, 0, sizeof(p));
+    p.n_linear = m->n_linear;
+    p.K0 = a.D + a.C;
+    p.KB0 = pk->layers[0].Kp / 64;
+    p.H = m->dims[1];
+    p.nch_hidden = p.H / 128;
+    p.D = a.D; p.C = a.C;
+    p.n_last_chunks = (a.D + DPC - 1) / DPC;
+    p.n_terms = pk->n_terms;
+    p.M = (int)a.B;
+    p.act = m->act;
+    p.x = a.x; p.ldx = a.ldx; p.c = a.c; p.ldc = a.ldc;
+    p.y = a.y; p.ldy = a.ldy; p.ladj = a.ladj; p.accumulate = a.accumulate;
+    p.log_prob = a.log_prob; p.base_loc = a.base_loc; p.base_scale = a.base_scale;
+    p.bound = a.bound;
+    const float absL = fabsf(logf(a.slope));
+    p.aw = 2.f / absL;
+    p.ad = 1.f / absL;
+    p.dbg = g_timeline;
+    p.sched = wp.sched;
+    p.n_items = wp.n_items;
+    const bool x_ok = (a.ldx % 4 == 0) && (a.D % 4 == 0) && (((uintptr_t)a.x) % 16 == 0);
+    const bool c_ok = (a.C == 0) || ((a.C % 4 == 0) && (((uintptr_t)a.c) % 16 == 0) && (a.ldc % 4 == 0));
+    p.in_vec = (x_ok && c_ok) ? 1 : 0;
+    for (int l = 0; l < m->n_linear; ++l) { p.mapW[l] = wp.maps[l]; p.rd_mask[l] = wp.rd_mask[l]; }
+}
+
+// Lays out the shared-memory copy of `bias_room` floats: the base table (log_prob only), the bias of the
+// OUTPUT layer (47 reads per dim and thread) and as many hidden-layer biases as still fit, each 16-byte
+// aligned; the others are read from global memory.  `floats`: how many floats the copy takes.
+template <class Params>
+zk_status pair_place_biases(Params& p, const zk_mlp* m, const FusedLayerArgs& a, uint32_t bias_room,
+                            const char* what, uint32_t& floats) {
+    const TcPack* pk = (const TcPack*)m->tc;
+    const int L = m->n_linear;
+    int off = 0;
+    const int base_floats = a.log_prob ? ((3 * a.D + 3) & ~3) : 0;
+    ZK_REQUIRE((uint32_t)base_floats <= bias_room, "%s: no shared memory left for the base table", what);
+    bias_room -= (uint32_t)base_floats;
+    auto place = [&](int l) {
+        const int len = (m->dims[l + 1] + 3) & ~3;
+        p.bias[l] = pk->fused.bias[l];
+        p.bias_len[l] = m->dims[l + 1];
+        if ((uint32_t)(off + len) <= bias_room) { p.bias_off[l] = off; off += len; }
+        else p.bias_off[l] = -1;
+    };
+    place(L - 1);
+    for (int l = 0; l < L - 1; ++l) place(l);
+    for (int l = L; l < ZK_FUSED_MAX_LINEAR; ++l) { p.bias[l] = nullptr; p.bias_off[l] = -1; p.bias_len[l] = 0; }
+    p.base_off = off;
+    floats = (uint32_t)(off + base_floats);
+    return ZK_OK;
 }
 
 

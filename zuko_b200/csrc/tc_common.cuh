@@ -143,8 +143,8 @@ struct FusedPack {
     int n_items = 0;
     double issued_macs_per_row = 0;  // MACs the schedule issues per sample row (all split terms), bench bookkeeping
 };
-// the wide fused kernel's pack (fused_wide.cu): it shares FusedPack's permuted planes / biases
-// (fused.w, fused.bias) and adds its own tensor maps and issue schedule
+// the pack of a CTA-pair fused kernel (fused_wide.cu, fused_dual.cu): it shares FusedPack's permuted
+// planes / biases (fused.w, fused.bias) and adds its own tensor maps and issue schedule
 struct WidePack {
     bool ready = false;
     int uni = 0, bins = 0, D = 0, C = 0;
@@ -153,6 +153,10 @@ struct WidePack {
     int n_items = 0;
     uint8_t rd_mask[8] = {0, 0, 0, 0, 0, 0, 0, 0};  // per layer: K blocks of the A operand the layer reads
     double issued_macs_per_row = 0;  // MACs the schedule issues per sample row (all split terms)
+    // holds a schedule (one that passed its dry run) for this bijector
+    bool built_for(int univariate, int bins_, int D_, int C_) const {
+        return ready && uni == univariate && bins == bins_ && D == D_ && C == C_;
+    }
 };
 struct TcPack {
     std::vector<TcLayer> layers;
